@@ -56,6 +56,8 @@ class Linear(Module):
     def __init__(self, input_dims, output_dims, bias=True):
         super().__init__()
         s = 1.0 / math.sqrt(input_dims)
+        # tests/test_oracle_golden.py::attn_proj_weights replays this draw (order, bound, dtype) instead of storing
+        # the golden FlashAttention weights: change both together and regenerate tests/golden/reference_vectors.npz
         self.weight = mx.array(_np.random.uniform(-s, s, (output_dims, input_dims)).astype(_np.float32))
         if bias:
             self.bias = mx.array(_np.random.uniform(-s, s, (output_dims,)).astype(_np.float32))

@@ -1,13 +1,15 @@
 """Generates tests/golden/reference_vectors.npz by RUNNING THE REFERENCE'S OWN PYTHON.
 
-The reference (/root/reference, read-only) is pure Python over mlx.core; mlx==0.25.0 cannot be
-installed here.  This script puts oracle/mlx_numpy_shim (a float32 NumPy stand-in for the handful
-of mlx primitives involved) on sys.path, imports the reference's modules unmodified, feeds them
-seeded inputs and records inputs + outputs.  tests/test_oracle_golden.py then checks
-oracle/reference_math.py against these vectors, and the -m gpu tests check the CUDA path against
-them too.  Run only in the build container:
+The reference is pure Python over mlx.core (mlx==0.25.0), which this project does not depend on.  This script
+puts oracle/mlx_numpy_shim (a float32 NumPy stand-in for the handful of mlx primitives involved) on
+sys.path, imports the reference's modules unmodified, feeds them seeded inputs and records inputs +
+outputs.  tests/test_oracle_golden.py then checks oracle/reference_math.py against these vectors, and
+the -m gpu tests check the CUDA path against them too.  Run with a checkout of the reference:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
+
+The FlashAttention projection weights are not stored, which keeps the file under 1 MB: tests regenerate them
+from the seed set before each FlashAttention is built (tests/test_oracle_golden.py, attn_proj_weights).
 
 What is exercised (reference file:line):
   optimizers/muon.py:54-83     Muon.zeropower_via_newtonschulz5        (wide, tall, square, batched)
@@ -32,20 +34,23 @@ What is exercised (reference file:line):
 """
 import os
 import sys
+import tempfile
 from pathlib import Path
 
 import numpy as np
 
 HERE = Path(__file__).resolve().parent
 REPO = HERE.parents[1]
-REF = Path("/root/reference")
+if len(sys.argv) != 2:
+    raise SystemExit("usage: python tests/golden/make_golden.py <reference checkout>")
+REF = Path(sys.argv[1]).resolve()
 
 # the reference's package names (optimizers, arch, core) collide with this repo's drop-in shims:
 # make sure only the reference and the mlx shim are importable
 sys.path = [p for p in sys.path if p not in ("", str(REPO)) and Path(p or ".").resolve() != REPO]
 sys.path.insert(0, str(REF))
 sys.path.insert(0, str(REPO / "oracle" / "mlx_numpy_shim"))
-os.chdir("/tmp")
+os.chdir(tempfile.gettempdir())
 
 import mlx.core as mx  # noqa: E402  (the shim)
 import mlx.nn as nn  # noqa: E402
@@ -117,7 +122,7 @@ out["graft_out"] = np.asarray(sh._apply_grafting(mx.array(gu), mx.array(su)))
 S = 16
 mask = np.triu(np.full((S, S), -np.inf, dtype=np.float32), k=1)[None, None]
 for tag, (H, Hk) in (("mha", (4, 4)), ("mqa", (4, 1)), ("gqa", (4, 2))):
-    np.random.seed(7)
+    np.random.seed(7)           # the only draws from this seed are the q/k/v/o_proj weights (not stored)
     attn = FlashAttention(hidden_size=128, num_heads=H, num_kv_heads=Hk, head_dim=32)
     q, k, v = f32(2, S, H, 32), f32(2, S, Hk, 32), f32(2, S, Hk, 32)
     out[f"attn_{tag}_q"], out[f"attn_{tag}_k"], out[f"attn_{tag}_v"] = q, k, v
@@ -125,8 +130,6 @@ for tag, (H, Hk) in (("mha", (4, 4)), ("mqa", (4, 1)), ("gqa", (4, 2))):
     out[f"attn_{tag}_nomask"] = np.asarray(attn._flash_attention(mx.array(q), mx.array(k), mx.array(v), None))
     x = f32(2, S, 128)
     out[f"attn_{tag}_x"] = x
-    for nm in ("q_proj", "k_proj", "v_proj", "o_proj"):
-        out[f"attn_{tag}_{nm}"] = np.asarray(getattr(attn, nm).weight)
     out[f"attn_{tag}_call"] = np.asarray(attn(mx.array(x), mask=mx.array(mask)))
 
 # ---- RMSNorm / MLP / whole model ----------------------------------------------------------------

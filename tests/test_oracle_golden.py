@@ -63,6 +63,19 @@ def test_shampoo_statistics_preconditioning_grafting(golden):
     assert rel((su * (gu.norm() / su.norm())).numpy(), golden["graft_out"]) < RTOL
 
 
+def attn_proj_weights(H, Hk, D=32, hidden=128):
+    """q/k/v/o_proj weights of the FlashAttention tests/golden/make_golden.py built: mlx's Linear init (uniform in
+    +-1/sqrt(fan_in)), drawn in construction order from NumPy's legacy generator seeded with 7.  Regenerated here
+    rather than stored; a wrong draw fails the `attn_*_call` comparison below."""
+    rs = np.random.RandomState(7)
+    w = {}
+    for n, (fan_out, fan_in) in (("q", (H * D, hidden)), ("k", (Hk * D, hidden)), ("v", (Hk * D, hidden)),
+                                 ("o", (hidden, H * D))):
+        s = 1.0 / np.sqrt(fan_in)
+        w[n] = t(rs.uniform(-s, s, (fan_out, fan_in)).astype(np.float32))
+    return w
+
+
 def test_attention_matches_reference(golden):
     S = 16
     mask = R.causal_mask(S)
@@ -76,10 +89,11 @@ def test_attention_matches_reference(golden):
         lin = torch.nn.functional.linear
         H = 4
         Hk = k.shape[2]
-        qq = lin(x, t(golden[f"attn_{tag}_q_proj"])).reshape(2, S, H, 32)
-        kk = lin(x, t(golden[f"attn_{tag}_k_proj"])).reshape(2, S, Hk, 32)
-        vv = lin(x, t(golden[f"attn_{tag}_v_proj"])).reshape(2, S, Hk, 32)
-        y = lin(R.attention(qq, kk, vv, scale, mask).reshape(2, S, H * 32), t(golden[f"attn_{tag}_o_proj"]))
+        w = attn_proj_weights(H, Hk)
+        qq = lin(x, w["q"]).reshape(2, S, H, 32)
+        kk = lin(x, w["k"]).reshape(2, S, Hk, 32)
+        vv = lin(x, w["v"]).reshape(2, S, Hk, 32)
+        y = lin(R.attention(qq, kk, vv, scale, mask).reshape(2, S, H * 32), w["o"])
         assert rel(y.numpy(), golden[f"attn_{tag}_call"]) < RTOL, tag
 
 
